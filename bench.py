@@ -4,6 +4,7 @@ forward + backward, all 4 decoder scales) of Monodepth2.jl training.
 
   python bench.py --gpus N --steps K --warmup W          # this repo's CUDA path
   python bench.py --impl reference --gpus N --steps K    # the reference's CPU path (oracle port)
+  python bench.py --steps K --dump-outputs DIR           # also write the last timed step's loss and gradients (DIR/*.npy)
 
 A "step" is one pass of the hot path over one synthetic batch.  Workload at every N:
 BASELINE.json configs[1] -- 416x128, batch 8 per GPU, C=1 (KITTI gray as in train()),
@@ -159,6 +160,30 @@ def make_sets(n_sets, dev, seed0, smooth=False):
     return sets, base
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, st, grad_x):
+    """writes what md2_view_synthesis_loss_fwdbwd handed back for the input set `st` as float32 DIR/<name>.npy, named after
+    the md2_vsl_desc fields: loss, grad_disparity_<scale>, grad_rot_<source>, grad_trans_<source>, grad_source_<source>
+    (the inputs are seeded, so two builds run with the same arguments can be compared output for output)"""
+    import numpy as np
+    arrays = {"loss": st["loss"]}
+    arrays.update({f"grad_disparity_{l}": g for l, g in enumerate(st["gd"])})
+    for s, frame in enumerate((0, 2)):      # the source frames of desc_for
+        arrays[f"grad_rot_{s}"], arrays[f"grad_trans_{s}"] = st["gr"][s], st["gt"][s]
+        if grad_x:
+            arrays[f"grad_source_{s}"] = st["gx"][:, frame]
+    host = {k: v.float().cpu().numpy() for k, v in arrays.items()}
+    nbytes = sum(a.nbytes for a in host.values())
+    if nbytes > DUMP_MAX_BYTES:
+        raise SystemExit(f"--dump-outputs: {nbytes} B of outputs exceed the {DUMP_MAX_BYTES} B limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in host.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+    print(f"wrote {len(host)} outputs ({nbytes / 1e6:.1f} MB) to {out_dir}", file=sys.stderr)
+
+
 def run_ours(args):
     import monodepth2_jl_b200 as M
     from monodepth2_jl_b200 import _lib as L
@@ -200,6 +225,7 @@ def run_ours(args):
     n_sets = max(4, int(2.5 * l2_bytes / set_bytes) + 1)
     sets, base = make_sets(n_sets, dev, 42 + rank)
     # (automasking: the map is formed INSIDE the timed call, desc.compute_automask -- the per-step pre-pass of src/Monodepth.jl:159-164)
+    grad_x = not os.environ.get("MD2_BENCH_G0")
 
     def desc_for(st):
         x = st["x"]
@@ -208,7 +234,7 @@ def run_ours(args):
             disparities=st["disps"], K_cm=K_cm, invK_cm=invK_cm, rot=st["rv"], trans=st["tv"], pose_mode=1,
             invert=[1, 0], automask=None, compute_automask=AM, smooth_weight=sw, loss_scale=1.0 / LS, normalize_disparity=True, loss=st["loss"],
             grad_disparity=st["gd"], grad_rot=st["gr"], grad_trans=st["gt"],
-            grad_source=(None if os.environ.get("MD2_BENCH_G0") else [st["gx"][:, 0], st["gx"][:, 2]]), zero_grad_source=True, shape=(NB, CH, H_, W_))
+            grad_source=([st["gx"][:, 0], st["gx"][:, 2]] if grad_x else None), zero_grad_source=True, shape=(NB, CH, H_, W_))
 
     descs = [desc_for(st) for st in sets]
     lib, handle = ctx.lib, ctx.handle
@@ -251,6 +277,9 @@ def run_ours(args):
     sampler.sample()
     sampler.stop_flag = True
     launches = ctx.launches - l0
+    if args.dump_outputs and rank == 0:
+        # (now: the sections below run the same ring slots again and overwrite their outputs)
+        dump_outputs(args.dump_outputs, sets[(args.steps - 1) % n_sets], grad_x)
     from monodepth2_jl_b200 import dist as D
     ms = D.max_over_ranks(e0.elapsed_time(e1), device=dev)   # device time, max over ranks
     frames = NB * world * args.steps
@@ -725,7 +754,11 @@ def main():
     ap.add_argument("--no-train-step", action="store_true", help="skip the training-step section")
     ap.add_argument("--train-steps", type=int, default=30, help="timed steps of the training-step section")
     ap.add_argument("--tf32", action="store_true", help="allow TF32 in the stand-in model's convolutions (default: strict fp32)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the loss and gradients of the last timed "
+                    "step as float32 DIR/<name>.npy (CUDA arm, configs 2-4)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.config == 1):
+        ap.error("--dump-outputs writes the outputs of the CUDA view-synthesis loss path (--impl ours, --config 2, 3 or 4)")
     if args.config == 1:
         if int(os.environ.get("RANK", "0")) == 0:
             run_config1(args)

@@ -9,8 +9,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(CSRC, "_obj")
 LIB = os.path.join(CSRC, "libmd2_b200.so")
-SOURCES = ["md2_fused.cu", "md2_march_inst.cu", "md2_ops.cu", "md2_host.cu", "md2_optim.cu"]
-HEADERS = ["md2_math.cuh", "md2_fused.cuh", "md2_march.cuh", "md2_march2.cuh", "md2_common.cuh", "md2_launch.cuh",
+SOURCES = ["md2_fused.cu", "md2_ops.cu", "md2_host.cu", "md2_optim.cu"]
+HEADERS = ["md2_math.cuh", "md2_fused.cuh", "md2_march.cuh", "md2_march2.cuh", "md2_common.cuh",
            os.path.join("..", "..", "include", "md2.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--cudart", "shared", "-split-compile", "0"]
@@ -24,12 +24,14 @@ def _mtime(f):
 def build(force=False, verbose=False):
     nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
     extra = os.environ.get("MD2_NVCC_EXTRA", "").split()   # tuning experiments, e.g. -DMD2_PREFETCH=0
-    sources = [s for s in SOURCES if os.path.exists(os.path.join(CSRC, s))]
+    missing = [f for f in SOURCES + HEADERS if not os.path.exists(os.path.join(CSRC, f))]
+    if missing:
+        raise RuntimeError(f"nvcc build: missing source files {missing}")
     tag = hashlib.sha1(" ".join(NVCC_FLAGS + extra).encode()).hexdigest()[:10]    # objects of other flag sets are not reused
     os.makedirs(OBJ, exist_ok=True)
     hdr_t = max(_mtime(h) for h in HEADERS)
     objs, todo = [], []
-    for s in sources:
+    for s in SOURCES:
         o = os.path.join(OBJ, f"{os.path.splitext(s)[0]}.{tag}.o")
         objs.append(o)
         if force or not os.path.exists(o) or os.path.getmtime(o) < max(_mtime(s), hdr_t):
