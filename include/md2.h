@@ -13,7 +13,7 @@
  *    through md2_last_error() (thread-local).  Nothing throws or exits.
  *  - every tensor argument is a caller-owned DEVICE pointer to contiguous float32 in
  *    Julia (column-major) memory order: image (W,H,C,N), disparity (W,H,1,N), points
- *    (3,P,N) with p = (h-1)W + (w-1), grid (2,W,H,N), K/invK (3,3), R (3,3,N), t (3,1,N),
+ *    (3,P,N) with p = (h-1)W + (w-1), grid (2,W,H,N), K/invK (3,3) (or (3,3,N): md2_vsl_desc.per_image_K), R (3,3,N), t (3,1,N),
  *    rvec (3,N).  (W,H,C,N) column-major is bit-identical to row-major NCHW.
  *  - pixel coordinates are 1-based like the reference (src/utils.jl:47-51); frame indices
  *    passed through this ABI are 0-based.
@@ -180,6 +180,20 @@ typedef struct md2_vsl_desc {
      * sequence -- the reference's separate pre-pass folded into the call.  The map is a constant of the loss, as in the
      * reference (it is computed outside `gradient`). */
     int32_t compute_automask;
+    /* Camera intrinsics per image and their gradients (fields appended last: a zero-filled descriptor keeps one shared
+     * camera and computes no intrinsics gradient).
+     * per_image_K = 0: K / invK are one (3,3) pair for the batch; 1: K / invK are (3,3,N), element (i,j) of image n at
+     * K[9n + 3j + i] (like R in pose_mode 0).
+     * grad_K / grad_invK (nullable; OVERWRITTEN): dL/dK and dL/dinvK of the shape of K / invK -- (3,3) summed over sources
+     * and images for a shared camera, (3,3,N) summed over sources per image.  invK is an independent input, as in the
+     * reference (the call multiplies by the invK it is given; it never inverts K): dL/dK = sum G (R invK)^T + h t^T,
+     * dL/dinvK = sum (K R)^T G over the (source, image) pairs, with R, t the pose actually used (after composeT).
+     * Written by every call that writes grad_rot (value + gradient calls, the backward call, md2_warp_bwd); ignored by
+     * the forward-only calls.  The sums are taken in a fixed (image, source) order in double precision, so both
+     * gradients are bit-identical from run to run. */
+    int32_t per_image_K;
+    float* grad_K;
+    float* grad_invK;
 } md2_vsl_desc;
 
 int md2_view_synthesis_loss_fwd(md2_ctx*, const md2_vsl_desc*, md2_stream);
@@ -210,7 +224,7 @@ int md2_host_wait(md2_ctx*, int32_t lane);
  * W,H,N,C,S, source*, disparity[0], K, invK, pose_*, rot, trans, invert, min/max_depth;
  * out[s] contiguous (W,H,C,N). */
 int md2_warp_fwd(md2_ctx*, const md2_vsl_desc*, float* const* out, md2_stream);
-/* gout[s] (W,H,C,N) -> grad_disparity[0], grad_rot, grad_trans, grad_source (accumulated) */
+/* gout[s] (W,H,C,N) -> grad_disparity[0], grad_rot, grad_trans, grad_source (accumulated), grad_K / grad_invK (nullable) */
 int md2_warp_bwd(md2_ctx*, const md2_vsl_desc*, const float* const* gout, md2_stream);
 
 /* ---- F1  Flux.Optimise.update!(ADAM, ...)   call src/Monodepth.jl:165-171, src/simple_depth.jl:20,43 --------------
@@ -234,7 +248,9 @@ int md2_adam_step(md2_ctx*, int32_t n, float* const* params, const float* const*
  * disparity, rvec_0, tvec_0, rvec_1, tvec_1; loss_history (nullable, device, history_len floats) receives the
  * objective value of update number t at index t = clock[0] at that time (values beyond history_len are dropped).
  * One iteration is four launches captured once into a CUDA graph and replayed; the loop is ordered after the work
- * already enqueued on `stream` and before anything enqueued afterwards, and does not synchronise the host. */
+ * already enqueued on `stream` and before anything enqueued afterwards, and does not synchronise the host.
+ * per_image_K is accepted (N = 1 here); grad_K / grad_invK must be NULL (the intrinsics are not among the optimised
+ * tensors). */
 int md2_slow_depth(md2_ctx*, const md2_vsl_desc*, int32_t iters, float lr, float beta1, float beta2, float eps,
                    float* state, int64_t* clock, float* loss_history, int64_t history_len, md2_stream);
 

@@ -41,6 +41,8 @@ class VslDesc(C.Structure):
         ("zero_grad_source", C.c_int32),
         ("debug_choices", c_void),
         ("compute_automask", C.c_int32),
+        ("per_image_K", C.c_int32),
+        ("grad_K", c_void), ("grad_invK", c_void),
     ]
 
 
@@ -67,9 +69,10 @@ def make_vsl_desc(*, target, target_stride, sources, source_strides, disparities
                   pose_mode, invert, automask=None, min_depth=0.1, max_depth=100.0, smooth_weight, loss_scale,
                   normalize_disparity=True, loss=None, grad_disparity=None, grad_rot=None, grad_trans=None,
                   grad_source=None, viz_warped=None, viz_loss=None, saved=None, zero_grad_source=False, debug_choices=None,
-                  compute_automask=False, shape):
+                  compute_automask=False, per_image_K=False, grad_K=None, grad_invK=None, shape):
     """shape = (N, C, H, W).  `target`/`sources` are tensors whose data_ptr() is element
-    (n=0,c=0,y=0,x=0) of an (N,C,H,W) view with per-image stride *_stride and dense C,H,W."""
+    (n=0,c=0,y=0,x=0) of an (N,C,H,W) view with per-image stride *_stride and dense C,H,W.
+    per_image_K: K_cm / invK_cm hold N column-major (3,3) matrices (9 N floats) instead of one."""
     N, Cc, H, W = shape
     S, L = len(sources), len(disparities)
     if S > MAX_S or L > MAX_L:
@@ -113,6 +116,13 @@ def make_vsl_desc(*, target, target_stride, sources, source_strides, disparities
     d.saved = _ptr(saved)
     d.zero_grad_source = int(bool(zero_grad_source))
     d.compute_automask = int(bool(compute_automask))
+    nk = 9 * N if per_image_K else 9
+    for t, name in ((K_cm, "K"), (invK_cm, "invK"), (grad_K, "grad_K"), (grad_invK, "grad_invK")):
+        _chk(t, name)
+        if t is not None and t.numel() != nk:
+            raise ValueError(f"{name}: expected {nk} floats, got {t.numel()}")
+    d.per_image_K = int(bool(per_image_K))
+    d.grad_K, d.grad_invK = _ptr(grad_K), _ptr(grad_invK)
     if debug_choices is not None:
         if debug_choices.dtype != torch.int32 or not debug_choices.is_contiguous():
             raise TypeError("debug_choices: expected a contiguous int32 tensor")

@@ -22,7 +22,7 @@ struct Workspace {
 }  // namespace md2
 
 enum { MD2_WS_PARTIAL = 0, MD2_WS_SUMS, MD2_WS_POSE, MD2_WS_STATS, MD2_WS_DISP, MD2_WS_GDISP,
-       MD2_WS_MISC, MD2_WS_AUTOMASK, MD2_WS_COUNT };
+       MD2_WS_MISC, MD2_WS_AUTOMASK, MD2_WS_KGRAD, MD2_WS_COUNT };
 // workspace banks: calls that may be in flight at the same time must not share scratch.  Bank 0 serves the
 // device-pointer entry points (one stream at a time, md2.h), banks 1.. the lanes of the host-buffer entry point.
 enum { MD2_WS_BANKS = 1 + MD2_HOST_LANES };

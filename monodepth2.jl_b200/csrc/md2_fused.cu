@@ -628,6 +628,15 @@ __device__ __forceinline__ double warp_sum_d(double v) {
     return v;
 }
 
+// called once by every (source, image) after it wrote its row of k.part: true for the last of the S*N arrivals, which then
+// forms grad_K / grad_invK and resets the counter (so a replayed graph finds it at 0 again)
+__device__ __forceinline__ bool intrinsics_last(const IntrIO& k, int S, int N) {
+    __threadfence();
+    const bool last = atomicAdd(k.count, 1u) == (unsigned)(S * N - 1);
+    if (last) __threadfence();
+    return last;
+}
+
 constexpr int FIN_MAXROWS = 64;   // contributing full-resolution rows handled per pass of phase A
 constexpr int FIN_THREADS = 128;
 #ifndef MD2_FIN_MINB
@@ -641,7 +650,8 @@ constexpr int FIN_UNROLL = MD2_FIN_UNROLL;
 #define MD2_FIN_TIMING 0
 #endif  // small blocks: the whole grid is resident at once (one latency chain, no waves)
 
-__global__ void __launch_bounds__(FIN_THREADS, MD2_FIN_MINB) finish_kernel(const __grid_constant__ FusedParams p, int NP, int ipg, int bwd, int low_rows) {
+__global__ void __launch_bounds__(FIN_THREADS, MD2_FIN_MINB) finish_kernel(const __grid_constant__ FusedParams p, int NP, int ipg, int bwd, int low_rows,
+                                                                           const __grid_constant__ IntrIO intr) {
     extern __shared__ __align__(16) float vrow[];   // [W rounded up to 4] (adjoint blocks)
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     pdl_wait();
@@ -736,7 +746,25 @@ __global__ void __launch_bounds__(FIN_THREADS, MD2_FIN_MINB) finish_kernel(const
             pacc[0][threadIdx.x] = a;
         }
         __syncthreads();
-        if (threadIdx.x == 0 && MD2_FIN_TIMING != 1) finalize_pose(p.pose, s, nn, &pacc[0][0], &pacc[0][0] + 9);
+        __shared__ int last;
+        if (threadIdx.x == 0) {
+            last = 0;
+            if (MD2_FIN_TIMING != 1) {
+                finalize_pose(p.pose, s, nn, &pacc[0][0], &pacc[0][0] + 9);
+                if (intr.part) {   // (a separate kernel parameter: FusedParams, which the marching kernels read, keeps its layout)
+                    intrinsics_part(p.pose, s, nn, &pacc[0][0], &pacc[0][0] + 9, intr.part + 18 * (long long)b);
+                    last = intrinsics_last(intr, p.S, p.N);
+                }
+            }
+        }
+        if (intr.part) {   // (uniform: a launch parameter) the last pose block sums the intrinsics gradients, one element per thread
+            __syncthreads();
+            if (!last) return;
+            const int ne = 18 * (p.pose.kstride ? p.N : 1);
+            for (int e = threadIdx.x; e < ne; e += blockDim.x) reduce_intrinsics_elem(intr, p.pose.kstride, p.S, p.N, e);
+            __syncthreads();
+            if (threadIdx.x == 0) *intr.count = 0u;
+        }
         return;
     }
     b -= p.S * p.N;
@@ -1095,7 +1123,8 @@ static int check_desc(const md2_vsl_desc* d, bool need_loss_inputs) {
     MD2_REQUIRE(d->N >= 1, "N must be >= 1");
     MD2_REQUIRE(d->C == 1 || d->C == 3, "C must be 1 or 3");
     MD2_REQUIRE(d->S >= 1 && d->S <= MAX_S, "S must be 1 or 2");
-    MD2_REQUIRE(d->K && d->invK, "K / invK are null");
+    MD2_REQUIRE(d->K && d->invK, "K / invK are null (grad_K / grad_invK need them too)");
+    MD2_REQUIRE(d->per_image_K == 0 || d->per_image_K == 1, "per_image_K must be 0 (one (3,3) K / invK) or 1 ((3,3,N))");
     for (int s = 0; s < d->S; ++s) {
         MD2_REQUIRE(d->source[s] != nullptr, "null source image");
         MD2_REQUIRE(d->rot[s] && d->trans[s], "null pose");
@@ -1118,6 +1147,7 @@ static int check_desc(const md2_vsl_desc* d, bool need_loss_inputs) {
 static void fill_pose_io(const md2_vsl_desc* d, PoseIO& io) {
     io.mode = d->pose_mode;
     io.K = d->K; io.invK = d->invK;
+    io.kstride = d->per_image_K ? 9 : 0;
     for (int s = 0; s < MAX_S; ++s) {
         io.rot[s] = s < d->S ? d->rot[s] : nullptr;
         io.trans[s] = s < d->S ? d->trans[s] : nullptr;
@@ -1125,6 +1155,21 @@ static void fill_pose_io(const md2_vsl_desc* d, PoseIO& io) {
         io.grot[s] = s < d->S ? d->grad_rot[s] : nullptr;
         io.gtrans[s] = s < d->S ? d->grad_trans[s] : nullptr;
     }
+}
+
+// scratch of the intrinsics gradients in the ctx workspace of the current bank: arrival counter (16 bytes, zeroed when the
+// slot is allocated; the reducing thread leaves it at 0) | (S*N, 18) doubles.  All null when no intrinsics gradient is asked.
+static int intrinsics_io(md2_ctx* ctx, const md2_vsl_desc* d, IntrIO& k, cudaStream_t st) {
+    memset(&k, 0, sizeof(k));
+    if (!d->grad_K && !d->grad_invK) return 0;
+    const int64_t gen = ctx->ws_gen[ctx->bank];
+    char* buf = (char*)ws_get(ctx, MD2_WS_KGRAD, 16 + sizeof(double) * 18 * (size_t)d->S * d->N);
+    if (!buf) return 1;
+    if (ctx->ws_gen[ctx->bank] != gen) MD2_CHECK(cudaMemsetAsync(buf, 0, 16, st));
+    k.gK = d->grad_K; k.giK = d->grad_invK;
+    k.count = reinterpret_cast<unsigned*>(buf);
+    k.part = reinterpret_cast<double*>(buf + 16);
+    return 0;
 }
 
 enum { MODE_FWD = 0, MODE_BWD = 1, MODE_FWDBWD = 2 };
@@ -1220,6 +1265,9 @@ int run_vsl(md2_ctx* ctx, const md2_vsl_desc* d, int mode, float gloss, cudaStre
     p.loss = (mode == MODE_BWD) ? nullptr : d->loss;
     p.prep_part = do_stats ? part2 : nullptr;
     p.prep_nblk = prep_nblk;
+    IntrIO intr;
+    memset(&intr, 0, sizeof(intr));
+    if (bwd && intrinsics_io(ctx, d, intr, st)) return 1;
 
     cudaEvent_t evp0 = nullptr, evp3 = nullptr;   // profile mode 2: the step's first and last time stamp
     if (ctx->prof_on == 2) {
@@ -1274,7 +1322,7 @@ int run_vsl(md2_ctx* ctx, const md2_vsl_desc* d, int mode, float gloss, cudaStre
     if (ev1) MD2_CHECK(cudaEventRecord(ev1, st));
     {   // loss / statistics, pose gradients, adjoint of the upsample for the low-res decoder scales
         const int blocks = 1 + (bwd ? S * N + low_rows * N : 0);
-        MD2_CHECK(launch_after(2, finish_kernel, dim3(blocks), dim3(FIN_THREADS), sizeof(float) * ((W + 3) & ~3), st, p, NP, tiles, bwd ? 1 : 0, low_rows));
+        MD2_CHECK(launch_after(2, finish_kernel, dim3(blocks), dim3(FIN_THREADS), sizeof(float) * ((W + 3) & ~3), st, p, NP, tiles, bwd ? 1 : 0, low_rows, intr));
         MD2_LAUNCH_CHECK(ctx);
     }
     if (evp3) MD2_CHECK(cudaEventRecord(evp3, st));
@@ -1409,7 +1457,7 @@ __global__ void pose_prep_kernel(PoseIO io, int S, int N, float* __restrict__ po
     prepare_pose_one(io, i / N, i % N, pose_ab + (long long)i * 12);
 }
 
-__global__ void pose_final_kernel(PoseIO io, int S, int N, int NP, const float* __restrict__ sums) {
+__global__ void pose_final_kernel(PoseIO io, IntrIO intr, int S, int N, int NP, const float* __restrict__ sums) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= S * N) return;
     const int s = i / N, n = i % N;
@@ -1418,6 +1466,13 @@ __global__ void pose_final_kernel(PoseIO io, int S, int N, int NP, const float* 
     for (int k = 0; k < 9; ++k) G[k] = su[k];
     for (int k = 0; k < 3; ++k) h[k] = su[9 + k];
     finalize_pose(io, s, n, G, h);
+    if (intr.part) {
+        intrinsics_part(io, s, n, G, h, intr.part + 18 * (long long)i);
+        if (intrinsics_last(intr, S, N)) {
+            reduce_intrinsics(intr, io.kstride, S, N);
+            *intr.count = 0u;
+        }
+    }
 }
 
 template <int C, int S>
@@ -1556,7 +1611,9 @@ static int run_warp(md2_ctx* ctx, const md2_vsl_desc* d, float* const* out, cons
     else warp_bwd_kernel<3, 2><<<g, 256, 0, st>>>(p, io);
     MD2_LAUNCH_CHECK(ctx);
     if (launch_reduce_partials(ctx, partial, sums, NP, nullptr, N, bpi, NP, st)) return 1;
-    pose_final_kernel<<<cdiv(S * N, 64), 64, 0, st>>>(p.pose, S, N, NP, sums);
+    IntrIO intr;
+    if (intrinsics_io(ctx, d, intr, st)) return 1;
+    pose_final_kernel<<<cdiv(S * N, 64), 64, 0, st>>>(p.pose, intr, S, N, NP, sums);
     MD2_LAUNCH_CHECK(ctx);
     return 0;
 }

@@ -3,6 +3,7 @@
 // loss assembly and the pose finalisation.  The hot kernel itself is md2_march.cuh.
 // Everything here is __host__ __device__ so that tests/emul can run the same code on the CPU.
 #pragma once
+#include <stddef.h>
 #include "md2_math.cuh"
 
 namespace md2 {
@@ -13,12 +14,23 @@ constexpr int NSTAT = 4;   // per (scale, image): warp sum, smooth-x sum, smooth
 
 struct PoseIO {            // pose inputs / gradient outputs, Julia memory order
     int mode;              // 0: rot = R (3,3,N) col-major, trans = t ; 1: rot = rvec (3,N), trans = tvec
+    int kstride;           // floats between the K / invK of consecutive images: 0 (one camera) or 9 (md2_vsl_desc.per_image_K)
     const float* rot[MAX_S];
     const float* trans[MAX_S];
     int invert[MAX_S];
-    const float* K; const float* invK;   // (3,3) col-major
+    const float* K; const float* invK;   // (3,3[,N]) col-major
     float* grot[MAX_S];
     float* gtrans[MAX_S];
+};
+// (kstride sits in what was the padding after `mode`: the layout of FusedParams, which the marching kernels read, is unchanged)
+static_assert(offsetof(PoseIO, rot) == 8 && sizeof(PoseIO) == 96, "PoseIO layout");
+
+// intrinsics gradients (md2_vsl_desc.grad_K / grad_invK): every (source, image) leaves its 18 double contributions in
+// `part`; the last to arrive (device arrival counter, reset by that last arrival) sums them in a fixed order
+struct IntrIO {
+    float* gK; float* giK;     // nullable outputs, the shape of K / invK
+    double* part;              // (S*N, 18): Kbar | Kinvbar row-major of (source s, image n) at row s*N + n
+    unsigned* count;           // arrival counter, 0 between launches
 };
 
 struct FusedParams {
@@ -242,11 +254,32 @@ MD2_HD float loss_from_stats(const float* stats, int W, int H, int N, int L, con
     return (float)(loss * loss_scale);
 }
 
+// K, invK of image n as row-major doubles
+MD2_HD void load_K(const PoseIO& io, int n, double* K, double* Ki) {
+    const float* Kn = io.K + io.kstride * n;     // (9 N < 2^31: N <= 65535)
+    const float* Kin = io.invK + io.kstride * n;
+    for (int i = 0; i < 3; ++i)
+        for (int j = 0; j < 3; ++j) { K[3 * i + j] = (double)Kn[3 * j + i]; Ki[3 * i + j] = (double)Kin[3 * j + i]; }
+}
+
+// K, invK of image n and the pose (R, t) actually used for (source s, image n): composeT applied
+MD2_HD void pose_used(const PoseIO& io, int s, int n, double* K, double* Ki, double* R, double* t) {
+    load_K(io, n, K, Ki);
+    if (io.mode == 0) {
+        for (int i = 0; i < 3; ++i)
+            for (int j = 0; j < 3; ++j) R[3 * i + j] = (double)io.rot[s][9 * n + 3 * j + i];
+        for (int k = 0; k < 3; ++k) t[k] = io.trans[s][3 * n + k];
+    } else {
+        double r[3], tv[3];
+        for (int k = 0; k < 3; ++k) { r[k] = io.rot[s][3 * n + k]; tv[k] = io.trans[s][3 * n + k]; }
+        compose_T(r, tv, io.invert[s], R, t);
+    }
+}
+
 // pose gradients of one (source, image) from the accumulated G|h of all scales
 MD2_HD void finalize_pose(const PoseIO& io, int s, int n, const double* G, const double* h) {
     double K[9], Ki[9];
-    for (int i = 0; i < 3; ++i)
-        for (int j = 0; j < 3; ++j) { K[3 * i + j] = (double)io.K[3 * j + i]; Ki[3 * i + j] = (double)io.invK[3 * j + i]; }
+    load_K(io, n, K, Ki);
     double Rub[9], tub[3];
     precompose_bwd(K, Ki, G, h, Rub, tub);
     if (io.mode == 0) {
@@ -266,20 +299,49 @@ MD2_HD void finalize_pose(const PoseIO& io, int s, int n, const double* G, const
     }
 }
 
+// the contributions of one (source, image) to the intrinsics gradients from the same G|h: Kbar | Kinvbar, 18 doubles
+// row-major.  (Not inlined on the device: it runs once per (source, image) and would otherwise add to the register
+// pressure of the kernels that call it.)
+#if defined(__CUDACC__)
+static __host__ __device__ __noinline__
+#else
+inline
+#endif
+void intrinsics_part(const PoseIO& io, int s, int n, const double* G, const double* h, double* kpart) {
+    double K[9], Ki[9], R[9], t[3];
+    pose_used(io, s, n, K, Ki, R, t);
+    precompose_intr_bwd(K, Ki, R, t, G, h, kpart, kpart + 9);
+}
+
+// element e of grad_K | grad_invK (e < 18 * (kstride ? N : 1)) from the (S*N, 18) contributions: per image (summed over
+// sources in source order) or, for a shared camera, over all pairs in (image, source) order; double sums, float outputs in
+// Julia column-major order.  Every element is independent: a block forms them in parallel, one thread each.
+MD2_HD void reduce_intrinsics_elem(const IntrIO& k, int kstride, int S, int N, int e) {
+    const int m = e / 18, q = e - 18 * m;
+    const int n0 = kstride ? m : 0, n1 = kstride ? m + 1 : N;
+    double a = 0.0;
+    for (int n = n0; n < n1; ++n)
+        for (int s = 0; s < S; ++s) {
+            const double* src = k.part + ((long long)s * N + n) * 18 + q;   // (written by other blocks of the launch)
+#if defined(__CUDA_ARCH__)
+            a += __ldcg(src);
+#else
+            a += *src;
+#endif
+        }
+    const int r = q % 9, i = r / 3, j = r % 3;
+    float* out = q < 9 ? k.gK : k.giK;
+    if (out) out[9 * m + 3 * j + i] = (float)a;
+}
+
+MD2_HD void reduce_intrinsics(const IntrIO& k, int kstride, int S, int N) {
+    for (int e = 0; e < 18 * (kstride ? N : 1); ++e) reduce_intrinsics_elem(k, kstride, S, N, e);
+}
+
 // [composeT] + pre-composition of one (source, image)
 MD2_HD void prepare_pose_one(const PoseIO& io, int s, int n, float* ab, float* eb = nullptr) {
     double K[9], Ki[9], R[9], t[3];
-    for (int i = 0; i < 3; ++i)
-        for (int j = 0; j < 3; ++j) { K[3 * i + j] = (double)io.K[3 * j + i]; Ki[3 * i + j] = (double)io.invK[3 * j + i]; }
-    if (io.mode == 0) {
-        for (int i = 0; i < 3; ++i)
-            for (int j = 0; j < 3; ++j) R[3 * i + j] = (double)io.rot[s][9 * n + 3 * j + i];
-        for (int k = 0; k < 3; ++k) t[k] = io.trans[s][3 * n + k];
-    } else {
-        double r[3], tv[3];
-        for (int k = 0; k < 3; ++k) { r[k] = io.rot[s][3 * n + k]; tv[k] = io.trans[s][3 * n + k]; }
-        compose_T(r, tv, io.invert[s], R, t);
-    }
+    pose_used(io, s, n, K, Ki, R, t);
     precompose(K, Ki, R, t, ab);
     if (eb) precompose_e(K, Ki, R, t, eb);
 }

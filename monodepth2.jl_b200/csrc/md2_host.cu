@@ -97,6 +97,7 @@ struct Carver {
 struct Mirror {
     float *tgt, *src[MAX_S], *disp[MAX_L], *K, *invK, *rot[MAX_S], *trans[MAX_S], *automask;
     float *loss, *gdisp[MAX_L], *grot[MAX_S], *gtrans[MAX_S], *gsrc[MAX_S];
+    float *gK, *giK;               // intrinsics gradients: (3,3,N) per image, or one (3,3) partial per image group
     float *small_in, *small_out;
     size_t small_in_floats, small_out_floats;
     bool xcontig;                  // frames travel as whole images of `xstride` floats starting at host pointer xbase
@@ -195,21 +196,26 @@ static size_t carve(const md2_vsl_desc* d, char* base, Mirror& m, int groups) {
     }
     if (d->automask && m.in_slab) m.automask = m.in_dev ? m.in_dev + (d->automask - m.in_lo) : nullptr;
     else m.automask = d->automask ? c.take(N * (size_t)d->W * d->H) : nullptr;
-    // small inputs: K, invK, then per source rot, trans
-    m.small_in_floats = 18 + (size_t)d->S * (pr + 3) * N;
+    // small inputs: K, invK (9 floats each, 9 N per image), then per source rot, trans
+    const size_t kf = d->per_image_K ? 9 * N : 9;
+    m.small_in_floats = 2 * kf + (size_t)d->S * (pr + 3) * N;
     m.small_in = c.take(m.small_in_floats);
-    m.K = m.small_in; m.invK = m.small_in ? m.small_in + 9 : nullptr;
-    // small outputs: per source grot, gtrans, then the partial losses
-    m.small_out_floats = (size_t)d->S * (pr + 3) * N + HOST_MAX_GROUPS;
+    m.K = m.small_in; m.invK = m.small_in ? m.small_in + kf : nullptr;
+    // small outputs: per source grot, gtrans, the partial losses, then grad_K | grad_invK (per image, or one partial
+    // per image group for a shared camera) when asked for
+    const size_t gkf = (d->grad_K || d->grad_invK) ? (d->per_image_K ? 9 * N : 9 * (size_t)HOST_MAX_GROUPS) : 0;
+    m.small_out_floats = (size_t)d->S * (pr + 3) * N + HOST_MAX_GROUPS + 2 * gkf;
     m.small_out = c.take(m.small_out_floats);
     for (int s = 0; s < MAX_S; ++s) {
         const bool on = s < d->S && m.small_in;
-        m.rot[s] = on ? m.small_in + 18 + (size_t)s * (pr + 3) * N : nullptr;
+        m.rot[s] = on ? m.small_in + 2 * kf + (size_t)s * (pr + 3) * N : nullptr;
         m.trans[s] = on ? m.rot[s] + (size_t)pr * N : nullptr;
         m.grot[s] = on ? m.small_out + (size_t)s * (pr + 3) * N : nullptr;
         m.gtrans[s] = on ? m.grot[s] + (size_t)pr * N : nullptr;
     }
     m.loss = m.small_out ? m.small_out + (size_t)d->S * (pr + 3) * N : nullptr;
+    m.gK = (m.loss && gkf) ? m.loss + HOST_MAX_GROUPS : nullptr;
+    m.giK = m.gK ? m.gK + gkf : nullptr;
     return c.off;
 }
 
@@ -292,7 +298,9 @@ static int enqueue(md2_ctx* ctx, HostPath* h, const md2_vsl_desc* d, const Mirro
             const size_t px = (size_t)d->disp_w[l] * d->disp_h[l];
             g.disparity[l] = m.disp[l] + n0 * px; g.grad_disparity[l] = m.gdisp[l] + n0 * px;
         }
-        g.K = m.K; g.invK = m.invK;
+        const size_t ko = d->per_image_K ? (size_t)9 * n0 : 0, go = d->per_image_K ? (size_t)9 * n0 : (size_t)9 * k;
+        g.K = m.K + ko; g.invK = m.invK + ko;
+        g.grad_K = d->grad_K ? m.gK + go : nullptr; g.grad_invK = d->grad_invK ? m.giK + go : nullptr;
         g.automask = m.automask ? m.automask + (size_t)n0 * W * H : nullptr;
         g.loss = m.loss + k; g.viz_loss = nullptr; g.saved = nullptr;
         g.loss_scale = d->loss_scale * (float)nk / (float)N;   // mean over the whole batch = sum of the group shares
@@ -347,6 +355,20 @@ static int collect(md2_ctx* ctx, int lane) {
     double loss = 0.0;
     for (int k = 0; k < h->pend_groups; ++k) loss += (double)q[k];
     *d->loss = (float)loss;
+    q += HOST_MAX_GROUPS;
+    if (d->grad_K || d->grad_invK) {   // per image: the rows as they are; shared: the group partials added in group order
+        const size_t gkf = d->per_image_K ? (size_t)9 * d->N : (size_t)9 * HOST_MAX_GROUPS;
+        float* outs[2] = {d->grad_K, d->grad_invK};
+        for (int w = 0; w < 2; ++w, q += gkf) {
+            if (!outs[w]) continue;
+            if (d->per_image_K) { memcpy(outs[w], q, sizeof(float) * 9 * d->N); continue; }
+            for (int e = 0; e < 9; ++e) {
+                double a = 0.0;
+                for (int k = 0; k < h->pend_groups; ++k) a += (double)q[9 * k + e];
+                outs[w][e] = (float)a;
+            }
+        }
+    }
     return 0;
 }
 
@@ -355,6 +377,7 @@ static int submit(md2_ctx* ctx, const md2_vsl_desc* d, float seed, int groups, i
     MD2_REQUIRE(d != nullptr, "null descriptor");
     MD2_REQUIRE(d->N >= 1 && d->S >= 1 && d->S <= MAX_S && d->L >= 1 && d->L <= MAX_L, "bad N / S / L");
     MD2_REQUIRE(d->target && d->K && d->invK && d->loss, "null target / K / invK / loss");
+    MD2_REQUIRE(d->per_image_K == 0 || d->per_image_K == 1, "per_image_K must be 0 or 1");
     MD2_REQUIRE(!d->saved && !d->viz_loss && !d->viz_warped[0] && !d->viz_warped[1], "saved / viz outputs are not supported by the host entry point");
     MD2_REQUIRE(!d->debug_choices, "debug_choices is not supported by the host entry point");
     for (int s = 0; s < d->S; ++s) MD2_REQUIRE(d->source[s] && d->rot[s] && d->trans[s], "null source / pose");
@@ -387,8 +410,9 @@ static int submit(md2_ctx* ctx, const md2_vsl_desc* d, float seed, int groups, i
     }
     {   // stage the small inputs: K, invK, per source rot, trans
         float* q = h->hsmall;
-        memcpy(q, d->K, 9 * sizeof(float)); memcpy(q + 9, d->invK, 9 * sizeof(float));
-        q += 18;
+        const size_t kf = d->per_image_K ? (size_t)9 * d->N : 9;
+        memcpy(q, d->K, kf * sizeof(float)); memcpy(q + kf, d->invK, kf * sizeof(float));
+        q += 2 * kf;
         for (int s = 0; s < d->S; ++s) {
             memcpy(q, d->rot[s], sizeof(float) * pr * d->N); q += (size_t)pr * d->N;
             memcpy(q, d->trans[s], sizeof(float) * 3 * d->N); q += (size_t)3 * d->N;

@@ -316,4 +316,19 @@ MD2_HD void precompose_bwd(const double* K, const double* Kinv, const double* G,
     for (int i = 0; i < 3; ++i) tub[i] = Kt[3 * i] * h[0] + Kt[3 * i + 1] * h[1] + Kt[3 * i + 2] * h[2];
 }
 
+// the same adjoint with respect to the intrinsics, K^-1 an independent input (R, t: the pose actually used)
+//   Kbar = G (R K^-1)^T + h t^T ,  Kinvbar = (K R)^T G
+MD2_HD void precompose_intr_bwd(const double* K, const double* Kinv, const double* R, const double* t, const double* G,
+                                const double* h, double* Kb, double* Kib) {
+    double RKi[9], RKit[9], KR[9], KRt[9];
+    mat3_mul(R, Kinv, RKi);
+    mat3_t(RKi, RKit);
+    mat3_mul(G, RKit, Kb);
+    for (int i = 0; i < 3; ++i)
+        for (int j = 0; j < 3; ++j) Kb[3 * i + j] += h[i] * t[j];
+    mat3_mul(K, R, KR);
+    mat3_t(KR, KRt);
+    mat3_mul(KRt, G, Kib);
+}
+
 }  // namespace md2

@@ -169,6 +169,8 @@ static int run_slow_depth(md2_ctx* ctx, const md2_vsl_desc* d, int iters, float 
     MD2_REQUIRE(iters >= 0, "iters must be >= 0");
     MD2_REQUIRE(d->L == 1 && d->disp_w[0] == d->W && d->disp_h[0] == d->H, "one full-resolution disparity (src/simple_depth.jl:8)");
     MD2_REQUIRE(d->pose_mode == 1, "poses are (rvec, tvec) parameters: pose_mode must be 1");
+    MD2_REQUIRE(!d->grad_K && !d->grad_invK, "grad_K / grad_invK must be NULL: the intrinsics are not among the optimised tensors");
+    MD2_REQUIRE(d->per_image_K == 0 || d->per_image_K == 1, "per_image_K must be 0 or 1");
     MD2_REQUIRE(d->loss && d->grad_disparity[0], "loss / grad_disparity scratch is required");
     for (int s = 0; s < d->S; ++s) MD2_REQUIRE(d->grad_rot[s] && d->grad_trans[s], "grad_rot / grad_trans scratch is required");
     MD2_REQUIRE(!d->debug_choices && !d->saved && !d->viz_loss && !d->viz_warped[0] && !d->viz_warped[1], "debug / saved / viz outputs are not served here");

@@ -296,7 +296,10 @@ struct VslDesc
     zero_grad_source::Int32
     debug_choices::CuPtr{Int32}          # test hook of the C ABI; always NULL here
     compute_automask::Int32              # != 0 with automask == NULL: the call forms the automask map itself
+    per_image_K::Int32                   # 1: K / invK are (3,3,N), one camera per image
+    grad_K::P32; grad_invK::P32          # nullable: dL/dK, dL/dinvK (the shape of K / invK; invK an independent input)
 end
+per_image(K) = ndims(K) == 3 && size(K, 3) > 1
 pad(v, n, z) = ntuple(i -> i <= length(v) ? v[i] : z, n)
 frameptr(x::CuF, id) = pointer(x, (id - 1) * size(x, 1) * size(x, 2) * size(x, 3) + 1)   # x (W,H,C,L,N), 1-based frame id
 
@@ -304,17 +307,19 @@ frameptr(x::CuF, id) = pointer(x, (id - 1) * size(x, 1) * size(x, 2) * size(x, 3
     view_synthesis_loss(x, disparities, poses, K, invK; target_id, source_ids, scales, ...)
 
 Everything of `train_loss` after `model(...)` (src/training.jl:29-77) in three kernel launches.
-Returns `(loss::CuArray{Float32,1}, grads)` where `grads = (disparities, rvecs, tvecs)` are the
-gradients for a unit cotangent (the pullback scales them).
+Returns `(loss::CuArray{Float32,1}, grads)` where `grads = (disparities, rvecs, tvecs, K, invK)` are the
+gradients for a unit cotangent (the pullback scales them); the last two are `nothing` unless `grad_K`.
+K / invK are (3,3) for one camera or (3,3,N) for one camera per image.
 """
 function vsl_fwdbwd(x::CuF, disparities, rvecs, tvecs, K::CuF, invK::CuF; target_id, source_ids, scales,
                     min_depth, max_depth, disparity_smoothness, auto_loss = nothing, normalize = true,
-                    smooth_weight = nothing, loss_scale = nothing, viz = false, compute_automask = false)
+                    smooth_weight = nothing, loss_scale = nothing, viz = false, compute_automask = false, grad_K = false)
     W, H, C, Lf, N = size(x); S = length(source_ids); L = length(disparities)
     loss = CUDA.zeros(Float32, 1)
     gd = [similar(d) for d in disparities]; gr = [similar(r) for r in rvecs]; gt = [similar(t) for t in tvecs]
     vw = viz ? [CUDA.zeros(Float32, W, H, C, N) for _ in 1:S] : CuF[]
     vl = viz ? CUDA.zeros(Float32, W, H, 1, N) : nothing
+    gK = grad_K ? similar(K) : nothing; giK = grad_K ? similar(invK) : nothing
     sw = smooth_weight === nothing ? Float32[disparity_smoothness * s for s in scales[1:L]] : Float32.(smooth_weight)
     fs = Int64(W * H * C * Lf)
     desc = Ref(VslDesc(W, H, N, C, S, L, frameptr(x, target_id), fs,
@@ -327,12 +332,13 @@ function vsl_fwdbwd(x::CuF, disparities, rvecs, tvecs, K::CuF, invK::CuF; target
         Float32(loss_scale === nothing ? 1 / L : loss_scale), Int32(normalize), ptr(loss),
         pad([ptr(g) for g in gd], MAX_L, P32(0)), pad([ptr(g) for g in gr], MAX_S, P32(0)),
         pad([ptr(g) for g in gt], MAX_S, P32(0)), pad(P32[], MAX_S, P32(0)),
-        pad([ptr(v) for v in vw], MAX_S, P32(0)), ptr(vl), P32(0), Int32(0), CuPtr{Int32}(0), Int32(compute_automask && auto_loss === nothing)))
-    GC.@preserve x disparities rvecs tvecs K invK auto_loss loss gd gr gt vw vl begin
+        pad([ptr(v) for v in vw], MAX_S, P32(0)), ptr(vl), P32(0), Int32(0), CuPtr{Int32}(0), Int32(compute_automask && auto_loss === nothing),
+        Int32(per_image(K)), ptr(gK), ptr(giK)))
+    GC.@preserve x disparities rvecs tvecs K invK auto_loss loss gd gr gt vw vl gK giK begin
         check(ccall((:md2_view_synthesis_loss_fwdbwd, LIB), Cint, (Ptr{Cvoid}, Ptr{VslDesc}, Cfloat, Ptr{Cvoid}),
                     ctx(), desc, 1f0, stream()))
     end
-    loss, (gd, gr, gt), vw, vl
+    loss, (gd, gr, gt, gK, giK), vw, vl
 end
 
 """
@@ -345,7 +351,7 @@ pipeline as a CUDA graph while the arrays stay the same.  `loss::Vector{Float32}
 are host arrays written in place.
 """
 function vsl_fwdbwd_host!(loss::Vector{Float32}, grads, x::Array{Float32,5}, disparities, rvecs, tvecs,
-                          K::Matrix{Float32}, invK::Matrix{Float32}; target_id, source_ids, scales, min_depth, max_depth,
+                          K::Array{Float32}, invK::Array{Float32}; target_id, source_ids, scales, min_depth, max_depth,
                           disparity_smoothness, normalize = true, groups = 2, lane = nothing)
     W, H, C, Lf, N = size(x); S = length(source_ids); L = length(disparities)
     gd, gr, gt = grads
@@ -362,7 +368,7 @@ function vsl_fwdbwd_host!(loss::Vector{Float32}, grads, x::Array{Float32,5}, dis
         Float32(1 / L), Int32(normalize), hp(loss),
         pad([hp(g) for g in gd], MAX_L, P32(0)), pad([hp(g) for g in gr], MAX_S, P32(0)),
         pad([hp(g) for g in gt], MAX_S, P32(0)), pad(P32[], MAX_S, P32(0)),
-        pad(P32[], MAX_S, P32(0)), P32(0), P32(0), Int32(1), CuPtr{Int32}(0), Int32(0)))
+        pad(P32[], MAX_S, P32(0)), P32(0), P32(0), Int32(1), CuPtr{Int32}(0), Int32(0), Int32(per_image(K)), P32(0), P32(0)))
     GC.@preserve x disparities rvecs tvecs K invK loss gd gr gt begin
         if lane === nothing          # synchronous: returns when every output is in host memory
             check(ccall((:md2_view_synthesis_loss_fwdbwd_host, LIB), Cint, (Ptr{Cvoid}, Ptr{VslDesc}, Cfloat, Cint),
@@ -385,11 +391,12 @@ function view_synthesis_loss(x, disparities, rvecs, tvecs, K, invK; kw...)
     CUDA.@allowscalar loss[1]
 end
 function rrule(::typeof(view_synthesis_loss), x, disparities, rvecs, tvecs, K, invK; kw...)
-    loss, (gd, gr, gt), _, _ = vsl_fwdbwd(x, disparities, rvecs, tvecs, K, invK; kw...)
+    loss, (gd, gr, gt, gK, giK), _, _ = vsl_fwdbwd(x, disparities, rvecs, tvecs, K, invK; kw..., grad_K = true)
     function pb(Δ)
         s = Float32(unthunk(Δ))
-        # cotangents of Vector-of-array arguments are plain Vectors of arrays (what Zygote accumulates into)
-        NoTangent(), NoTangent(), [s .* g for g in gd], [s .* g for g in gr], [s .* g for g in gt], NoTangent(), NoTangent()
+        # cotangents of Vector-of-array arguments are plain Vectors of arrays (what Zygote accumulates into);
+        # K and invK get theirs too (learned intrinsics), invK as an input of its own as in the reference
+        NoTangent(), NoTangent(), [s .* g for g in gd], [s .* g for g in gr], [s .* g for g in gt], s .* gK, s .* giK
     end
     (CUDA.@allowscalar loss[1]), pb
 end

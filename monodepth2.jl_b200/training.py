@@ -48,13 +48,29 @@ class TrainCache:
     scales: Sequence[float]
 
     def __post_init__(self):
-        # column-major copies handed to the C ABI, made once
-        self.K_cm = _cm(_f32c(self.K.reshape(3, 3)))
-        self.invK_cm = _cm(_f32c(self.invK.reshape(3, 3)))
+        # column-major copies handed to the C ABI, made once -- for a constant shared camera only: intrinsics that are
+        # learned (requires_grad) or given per image go through view_synthesis_loss's differentiable route at every call
+        fixed = not (self.K.requires_grad or self.invK.requires_grad) and self.K.numel() == 9 and self.invK.numel() == 9
+        self.K_cm = _cm(_f32c(self.K.reshape(3, 3))) if fixed else None
+        self.invK_cm = _cm(_f32c(self.invK.reshape(3, 3))) if fixed else None
 
 
 def _frame_ptr_view(x, idx):
     return x[:, idx]
+
+
+def _intrinsics(K, invK):
+    """K, invK of shape (3,3), (1,3,3) or (M,3,3) (natural maths convention) -> (K, invK) as (M,3,3) views, per_image"""
+    Kb, iKb = K.reshape(-1, 3, 3), invK.reshape(-1, 3, 3)
+    M = max(Kb.shape[0], iKb.shape[0])
+    if Kb.shape[0] not in (1, M) or iKb.shape[0] not in (1, M):
+        raise ValueError(f"K {tuple(K.shape)} and invK {tuple(invK.shape)}: expected (3,3), (1,3,3) or (N,3,3)")
+    return Kb.expand(M, 3, 3), iKb.expand(M, 3, 3), M > 1
+
+
+def _intrinsics_cm(Kb, per_image):
+    """(M,3,3) natural -> the C ABI's column-major block: one (3,3) for a shared camera, (3,3,M) per image"""
+    return _cm(_f32c(Kb.detach() if per_image else Kb.detach()[0]))
 
 
 class _ViewSynthesisLoss(torch.autograd.Function):
@@ -65,6 +81,10 @@ class _ViewSynthesisLoss(torch.autograd.Function):
     @staticmethod
     def forward(ctx, cfg, x, *tensors):
         Lc, S = cfg["L"], cfg["S"]
+        intr = cfg["grad_K"]                 # K, invK are the last two tensor inputs: gradients wanted
+        K_cm, invK_cm = cfg["K_cm"], cfg["invK_cm"]
+        if intr:
+            K_cm, invK_cm = (_intrinsics_cm(t, cfg["per_image_K"]) for t in tensors[-2:])
         disps = [_f32c(t) for t in tensors[:Lc]]
         rot = [_f32c(t) for t in tensors[Lc:Lc + S]]
         trans = [_f32c(t) for t in tensors[Lc + S:Lc + 2 * S]]
@@ -72,6 +92,8 @@ class _ViewSynthesisLoss(torch.autograd.Function):
         require_cuda(x, *disps, *rot, *trans)
         N, Lf, Cc, H, W = x.shape
         c = Context.get(x.device)
+        if cfg["per_image_K"] and K_cm.numel() != 9 * N:
+            raise ValueError(f"per-image K / invK: expected {N} matrices, got {K_cm.numel() // 9}")
         need = [ctx.needs_input_grad[2 + i] for i in range(len(tensors))]
         need_x = ctx.needs_input_grad[1] and cfg.get("grad_x", True)
         any_grad = any(need) or need_x
@@ -81,6 +103,8 @@ class _ViewSynthesisLoss(torch.autograd.Function):
         gr = [torch.empty_like(r) for r in rot] if any_grad else None
         gt = [torch.empty_like(t) for t in trans] if any_grad else None
         gx = torch.zeros_like(x) if need_x else None
+        gK = torch.empty_like(K_cm) if intr and need[-2] else None
+        giK = torch.empty_like(invK_cm) if intr and need[-1] else None
         viz_w = viz_l = None
         if cfg.get("viz"):
             viz_w = [torch.empty(N, Cc, H, W, device=dev, dtype=_F32) for _ in range(S)]
@@ -89,7 +113,8 @@ class _ViewSynthesisLoss(torch.autograd.Function):
         desc = L.make_vsl_desc(
             target=x[:, tid], target_stride=x.stride(0),
             sources=[x[:, i] for i in sid], source_strides=[x.stride(0)] * S,
-            disparities=disps, K_cm=cfg["K_cm"], invK_cm=cfg["invK_cm"], rot=rot, trans=trans,
+            disparities=disps, K_cm=K_cm, invK_cm=invK_cm, per_image_K=cfg["per_image_K"], grad_K=gK, grad_invK=giK,
+            rot=rot, trans=trans,
             pose_mode=cfg["pose_mode"], invert=cfg["invert"], automask=cfg.get("automask"),
             min_depth=cfg["min_depth"], max_depth=cfg["max_depth"], smooth_weight=cfg["smooth_weight"],
             loss_scale=cfg["loss_scale"], normalize_disparity=cfg["normalize"], loss=loss,
@@ -100,6 +125,10 @@ class _ViewSynthesisLoss(torch.autograd.Function):
         if any_grad:
             c.call("md2_view_synthesis_loss_fwdbwd", C.byref(desc), 1.0)
             ctx.grads = (gd, gr, gt, gx)
+            ctx.intr = None
+            if intr:   # column-major (3,3[,M]) -> natural (M,3,3), the shape of the tensor inputs
+                nat = lambda g: None if g is None else g.reshape(-1, 3, 3).transpose(1, 2)
+                ctx.intr = (nat(gK), nat(giK))
         else:
             c.call("md2_view_synthesis_loss_fwd", C.byref(desc))
             ctx.grads = None
@@ -114,7 +143,8 @@ class _ViewSynthesisLoss(torch.autograd.Function):
     def backward(ctx, g, *unused):
         gd, gr, gt, gx = ctx.grads
         scale = lambda t: None if t is None else t * g
-        return (None, scale(gx), *[scale(t) for t in gd], *[scale(t) for t in gr], *[scale(t) for t in gt])
+        intr = [scale(t) for t in ctx.intr] if ctx.intr is not None else []
+        return (None, scale(gx), *[scale(t) for t in gd], *[scale(t) for t in gr], *[scale(t) for t in gt], *intr)
 
 
 def view_synthesis_loss(x, disparities, rot, trans, K, invK, *, target_id=1, source_ids=(0, 2),
@@ -133,15 +163,23 @@ def view_synthesis_loss(x, disparities, rot, trans, K, invK, *, target_id=1, sou
     compute_automask=True (with auto_loss=None): the automask map is formed inside the call from the un-warped source
     frames (the pre-pass of src/Monodepth.jl:159-164 folded in; a constant of the loss, as in the reference).
     debug_choices: optional int32 (L,N,H,W,1+S) test hook that receives the kernel's discrete decisions
-    (include/md2.h: md2_vsl_desc.debug_choices)."""
+    (include/md2.h: md2_vsl_desc.debug_choices).
+    K, invK: (3,3) or (1,3,3) for one camera, (N,3,3) for a camera per image (a mix broadcasts).  invK is an input of its
+    own, as in the reference (it is never derived from K).  When either requires grad, both gradients flow back through
+    autograd; K_cm / invK_cm (pre-made column-major copies of a constant shared camera) are then ignored."""
     S, Lc = len(source_ids), len(disparities)
+    Kb, iKb, per_image = _intrinsics(K, invK)
+    grad_K = torch.is_grad_enabled() and (K.requires_grad or invK.requires_grad)
+    if grad_K or per_image:
+        K_cm = invK_cm = None
     if invert is None:
         invert = [sid < target_id for sid in source_ids]
     if not poses_are_rvec:
         rot = [_cm(r) for r in rot]
     cfg = dict(L=Lc, S=S, source_ids=list(source_ids), target_id=target_id,
-               K_cm=K_cm if K_cm is not None else _cm(_f32c(K.reshape(3, 3))),
-               invK_cm=invK_cm if invK_cm is not None else _cm(_f32c(invK.reshape(3, 3))),
+               K_cm=K_cm if K_cm is not None or grad_K else _intrinsics_cm(Kb, per_image),
+               invK_cm=invK_cm if invK_cm is not None or grad_K else _intrinsics_cm(iKb, per_image),
+               per_image_K=per_image, grad_K=grad_K,
                pose_mode=1 if poses_are_rvec else 0, invert=invert,
                automask=_f32c(auto_loss.detach()) if auto_loss is not None else None,
                min_depth=min_depth, max_depth=max_depth,
@@ -151,7 +189,7 @@ def view_synthesis_loss(x, disparities, rot, trans, K, invK, *, target_id=1, sou
                normalize=normalize_disparity, viz=return_viz, debug_choices=debug_choices,
                compute_automask=bool(compute_automask) and auto_loss is None)
     trans = [t.reshape(-1, 3) for t in trans]
-    out = _ViewSynthesisLoss.apply(cfg, x, *disparities, *rot, *trans)
+    out = _ViewSynthesisLoss.apply(cfg, x, *disparities, *rot, *trans, *((Kb, iKb) if grad_K else ()))
     if return_viz:
         loss, viz_l, *viz_w = out
         return loss, viz_w, viz_l
@@ -171,13 +209,15 @@ class HostViewSynthesisLoss:
     outputs are in `lane_grads[k]` and returns the loss, so the device-to-host copies of one step overlap the
     host-to-device copies and kernels of the next (md2_view_synthesis_loss_fwdbwd_host_submit / md2_host_wait).
 
-    x (N,3,C,H,W); disparities (N,1,h_i,w_i) per scale; rvecs / tvecs (N,3) per source; K, invK (3,3)."""
+    x (N,3,C,H,W); disparities (N,1,h_i,w_i) per scale; rvecs / tvecs (N,3) per source; K, invK (3,3) for one camera or
+    (N,3,3) per image.  grad_K=True: also d loss / d K and d loss / d invK, in grads["K"] / grads["invK"] (the shape of
+    K / invK, natural convention; views of pinned column-major buffers)."""
 
     LANES = 3
 
     def __init__(self, N, C_, H, W, disp_sizes, K, invK, *, device=None, target_id=1, source_ids=(0, 2),
                  scales=(0.125, 0.25, 0.5, 1.0), min_depth=0.1, max_depth=100.0, disparity_smoothness=1e-3,
-                 automask=False, normalize_disparity=True, grad_x=False, groups=2, lanes=1):
+                 automask=False, normalize_disparity=True, grad_x=False, groups=2, lanes=1, grad_K=False):
         dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         self.ctx = Context.get(dev)
         self.groups, self.S, self.L = int(groups), len(source_ids), len(disp_sizes)
@@ -194,8 +234,12 @@ class HostViewSynthesisLoss:
                 offs.append(tot); tot += (n + 63) & ~63
             buf = torch.zeros(tot, dtype=_F32).pin_memory()
             return [buf[o:o + n].view(*sh) for o, n, sh in zip(offs, sizes, shapes)], buf
-        self._K = _cm(_f32c(K.reshape(3, 3).cpu())).pin_memory()
-        self._invK = _cm(_f32c(invK.reshape(3, 3).cpu())).pin_memory()
+        Kb, iKb, per_image = _intrinsics(K.detach().cpu(), invK.detach().cpu())
+        if per_image and Kb.shape[0] != N:
+            raise ValueError(f"per-image K / invK: expected {N} matrices, got {Kb.shape[0]}")
+        self._K, self._invK = _intrinsics_cm(Kb, per_image).pin_memory(), _intrinsics_cm(iKb, per_image).pin_memory()
+        # (natural-convention view of a pinned column-major output buffer of the shape of K)
+        kview = lambda buf: buf.view(-1, 3, 3).transpose(1, 2) if per_image else buf.view(3, 3).t()
         self.lane_inputs, self.lane_grads, self._lane_loss, self._descs = [], [], [], []
         for _ in range(lanes):
             am_in = bool(automask) and automask != "inside"          # a map handed in by the caller ("inside": formed by the call)
@@ -206,6 +250,10 @@ class HostViewSynthesisLoss:
                           automask=big[1 + nd] if am_in else None, _slab=in_buf)
             grads = dict(disparities=gbig, rvecs=[pin(N, 3) for _ in source_ids],
                          tvecs=[pin(N, 3) for _ in source_ids], x=pin(N, 3, C_, H, W) if grad_x else None, _slab=out_buf)
+            gK_cm = pin(self._K.numel()) if grad_K else None
+            giK_cm = pin(self._invK.numel()) if grad_K else None
+            if grad_K:
+                grads.update(K=kview(gK_cm), invK=kview(giK_cm))
             loss = pin(1)
             x, gx = inputs["x"], grads["x"]
             desc = L.make_vsl_desc(
@@ -216,12 +264,13 @@ class HostViewSynthesisLoss:
                 smooth_weight=[disparity_smoothness * s for s in list(scales)[:self.L]], loss_scale=1.0 / self.L,
                 normalize_disparity=normalize_disparity, loss=loss, grad_disparity=grads["disparities"],
                 grad_rot=grads["rvecs"], grad_trans=grads["tvecs"],
-                grad_source=[gx[:, i] for i in source_ids] if grad_x else None, zero_grad_source=True, shape=(N, C_, H, W))
+                grad_source=[gx[:, i] for i in source_ids] if grad_x else None, zero_grad_source=True,
+                per_image_K=per_image, grad_K=gK_cm, grad_invK=giK_cm, shape=(N, C_, H, W))
             self.lane_inputs.append(inputs); self.lane_grads.append(grads); self._lane_loss.append(loss); self._descs.append(desc)
         self.inputs, self.grads, self._loss, self.desc = self.lane_inputs[0], self.lane_grads[0], self._lane_loss[0], self._descs[0]
         x = self.inputs["x"]
         self.h2d_bytes = 4 * sum(t.numel() for t in [x] + self.inputs["disparities"] + self.inputs["rvecs"] + self.inputs["tvecs"]
-                                 + ([self.inputs["automask"]] if self.inputs["automask"] is not None else [])) + 72
+                                 + ([self.inputs["automask"]] if self.inputs["automask"] is not None else [])) + 8 * self._K.numel()
         self.d2h_bytes = 4 + 4 * sum(t.numel() for t in self.grads["disparities"] + self.grads["rvecs"] + self.grads["tvecs"]) \
             + (8 * N * C_ * H * W if grad_x else 0)
 
@@ -276,7 +325,7 @@ class _Warp(torch.autograd.Function):
         desc = L.make_vsl_desc(
             target=None, target_stride=0, sources=[x[:, i] for i in cfg["source_ids"]],
             source_strides=[x.stride(0)] * S, disparities=[disp], K_cm=cfg["K_cm"], invK_cm=cfg["invK_cm"],
-            rot=rot, trans=trans, pose_mode=0, invert=[0] * S, min_depth=cfg["min_depth"],
+            per_image_K=cfg["per_image_K"], rot=rot, trans=trans, pose_mode=0, invert=[0] * S, min_depth=cfg["min_depth"],
             max_depth=cfg["max_depth"], smooth_weight=[0.0], loss_scale=1.0, shape=(N, Cc, H, W))
         arr = (C.c_void_p * S)(*[o.data_ptr() for o in outs])
         Context.get(x.device).call("md2_warp_fwd", C.byref(desc), arr)
@@ -299,7 +348,7 @@ class _Warp(torch.autograd.Function):
         desc = L.make_vsl_desc(
             target=None, target_stride=0, sources=[x[:, i] for i in cfg["source_ids"]],
             source_strides=[x.stride(0)] * S, disparities=[disp], K_cm=cfg["K_cm"], invK_cm=cfg["invK_cm"],
-            rot=rot, trans=trans, pose_mode=0, invert=[0] * S, min_depth=cfg["min_depth"],
+            per_image_K=cfg["per_image_K"], rot=rot, trans=trans, pose_mode=0, invert=[0] * S, min_depth=cfg["min_depth"],
             max_depth=cfg["max_depth"], smooth_weight=[0.0], loss_scale=1.0, grad_disparity=[gd], grad_rot=gr,
             grad_trans=gt, grad_source=[gx[:, i] for i in cfg["source_ids"]] if gx is not None else None,
             shape=(N, Cc, H, W))
@@ -316,8 +365,9 @@ def warp(disp, x, Ps, backprojections, projections, invKs, Ks, *, min_depth, max
     `backprojections` / `projections` are accepted for signature parity; the fused kernel
     derives the pixel grid itself."""
     S = len(source_ids)
-    cfg = dict(S=S, source_ids=list(source_ids), K_cm=_cm(_f32c(Ks.reshape(3, 3))),
-               invK_cm=_cm(_f32c(invKs.reshape(3, 3))), min_depth=float(min_depth), max_depth=float(max_depth))
+    Kb, iKb, per_image = _intrinsics(Ks, invKs)
+    cfg = dict(S=S, source_ids=list(source_ids), K_cm=_intrinsics_cm(Kb, per_image), invK_cm=_intrinsics_cm(iKb, per_image),
+               per_image_K=per_image, min_depth=float(min_depth), max_depth=float(max_depth))
     N = x.shape[0]
     disp = disp.reshape(N, 1, x.shape[-2], x.shape[-1])
     Rs = [P[0] for P in Ps]
