@@ -214,7 +214,8 @@ int md2_view_synthesis_loss_fwdbwd_host(md2_ctx*, const md2_vsl_desc* host_desc,
  * host memory.  The lanes own separate streams, staging buffers, scratch and cached graphs, so the device-to-host copies
  * of step i overlap the host-to-device copies and kernels of step i+1 (submit(i+1, lane B) before wait(lane A)).
  * With one image group (groups = 1), inputs that lie in ONE stretch of host memory (frames, every disparity, automask
- * carved out of one pinned allocation) travel as a single copy, and so do the disparity gradients on the way back.  The host
+ * carved out of one pinned allocation) travel as a single copy.  So do the disparity gradients on the way back when the
+ * L arrays lie back to back, with no gap between them; the call never writes a host byte outside its output arrays.  The host
  * buffers of a submitted descriptor must stay valid and untouched until its wait returns; submitting on a lane with an
  * uncollected call collects that call first.  md2_view_synthesis_loss_fwdbwd_host == submit + wait on lane 0. */
 int md2_view_synthesis_loss_fwdbwd_host_submit(md2_ctx*, const md2_vsl_desc* host_desc, float seed, int32_t groups, int32_t lane);

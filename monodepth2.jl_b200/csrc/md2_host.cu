@@ -105,7 +105,8 @@ struct Mirror {
     int64_t xspan;                 // floats from xbase to the end of the last frame in use of one image
     // slab mode (one image group): every large input / every disparity gradient lies in ONE stretch of host memory
     // (a caller that carves its pinned buffers out of one allocation): the device mirror keeps the host layout and the
-    // stretch travels as a single copy at the large-transfer rate of the link
+    // stretch travels as a single copy at the large-transfer rate of the link.  Inputs may leave small gaps between
+    // arrays (read, never written); the disparity gradients must lie back to back
     bool in_slab, out_slab;
     const float* in_lo; float* in_dev; size_t in_floats;
     float* out_lo; float* out_dev; size_t out_floats;
@@ -154,11 +155,13 @@ static size_t carve(const md2_vsl_desc* d, char* base, Mirror& m, int groups) {
         m.in_slab = one_stretch(p, n, cnt, 1024, &m.in_lo, &m.in_floats);
     }
     if (groups == 1 && d->L >= 2) {
+        // outputs: only gradient arrays that lie back to back qualify.  The stretch is copied back whole, so any gap
+        // between two arrays would be overwritten with the never-written device memory of its mirror.
         const float* p[MAX_L]; size_t n[MAX_L];
         bool all = true;
         for (int l = 0; l < d->L; ++l) { p[l] = d->grad_disparity[l]; n[l] = N * (size_t)d->disp_w[l] * d->disp_h[l]; all = all && p[l]; }
         const float* lo = nullptr;
-        m.out_slab = all && one_stretch(p, n, d->L, 1024, &lo, &m.out_floats);
+        m.out_slab = all && one_stretch(p, n, d->L, 0, &lo, &m.out_floats);
         m.out_lo = const_cast<float*>(lo);
     }
     m.in_dev = m.in_slab ? c.take(m.in_floats) : nullptr;

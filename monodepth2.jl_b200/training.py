@@ -225,13 +225,13 @@ class HostViewSynthesisLoss:
             raise ValueError(f"lanes must be in 1 .. {self.LANES}")
         pin = lambda *shape: torch.zeros(*shape, dtype=_F32).pin_memory()
 
-        def slab(shapes):
-            """tensors of the given shapes carved out of ONE pinned allocation (64-float alignment): the host entry point
-            recognises the stretch and moves it with a single copy at the large-transfer rate of the link"""
+        def slab(shapes, align=64):
+            """tensors of the given shapes carved out of ONE pinned allocation (`align`-float alignment): the host entry
+            point recognises the stretch and moves it with a single copy at the large-transfer rate of the link"""
             sizes = [int(torch.Size(sh).numel()) for sh in shapes]
             offs, tot = [], 0
             for n in sizes:
-                offs.append(tot); tot += (n + 63) & ~63
+                offs.append(tot); tot += (n + align - 1) // align * align
             buf = torch.zeros(tot, dtype=_F32).pin_memory()
             return [buf[o:o + n].view(*sh) for o, n, sh in zip(offs, sizes, shapes)], buf
         Kb, iKb, per_image = _intrinsics(K.detach().cpu(), invK.detach().cpu())
@@ -244,7 +244,9 @@ class HostViewSynthesisLoss:
         for _ in range(lanes):
             am_in = bool(automask) and automask != "inside"          # a map handed in by the caller ("inside": formed by the call)
             big, in_buf = slab([(N, 3, C_, H, W)] + [(N, 1, h, w) for (w, h) in disp_sizes] + ([(N, 1, H, W)] if am_in else []))
-            gbig, out_buf = slab([(N, 1, h, w) for (w, h) in disp_sizes])
+            # (the disparity gradients back to back: the one-copy return route takes only a stretch without gaps, and
+            # the kernels store these gradients as scalars, so they need no alignment)
+            gbig, out_buf = slab([(N, 1, h, w) for (w, h) in disp_sizes], align=1)
             nd = len(disp_sizes)
             inputs = dict(x=big[0], disparities=big[1:1 + nd], rvecs=[pin(N, 3) for _ in source_ids], tvecs=[pin(N, 3) for _ in source_ids],
                           automask=big[1 + nd] if am_in else None, _slab=in_buf)
